@@ -54,6 +54,36 @@ def measured_traffic(kernel):
         return None
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, rank=0, world=1):
+    """--dump-outputs: write what the timed path returned in its last step as ``<out_dir>/<name>.npy``.
+    Every array has one row per game; integers are stored as float64 (exact up to 2**53), 64-bit hashes
+    as two 32-bit halves.  When the rows exceed DUMP_LIMIT_BYTES a fixed, seeded sample of games is kept
+    (``game_index.npy`` names the rows in every case), so two builds can be compared file by file."""
+    conv = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype == np.uint64:
+            conv[name + "_hi"] = (a >> np.uint64(32)).astype(np.float64)
+            conv[name + "_lo"] = (a & np.uint64(0xFFFFFFFF)).astype(np.float64)
+        elif a.dtype.kind in "iub":
+            conv[name] = a.astype(np.float64)
+        else:
+            conv[name] = a.astype(np.float32)
+    G = len(next(iter(conv.values())))
+    row_bytes = sum(a[:1].nbytes for a in conv.values()) + 8
+    keep = np.arange(G)
+    if G * row_bytes > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(SEED).choice(G, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+    conv["game_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in conv.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a if name == "game_index" else a[keep])
+
+
 def measured_peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -278,6 +308,10 @@ def run_playout(args):
     t_wall = time.perf_counter() - t_wall0
     launches = gb.launch_count() - launches0
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
+    if args.dump_outputs:
+        r = gb.playout_results()  # what playout_stream() returns: in this mode "score" holds the games started
+        dump_outputs(args.dump_outputs, {"chk": r["chk"], "plies": r["plies"], "games": r["score"], "hash": r["hash"]},
+                     rank, world)
 
     # ---- e2e: the public call with host result buffers, wall clock ------------------------------
     barrier()
@@ -758,6 +792,13 @@ def run_selfplay(args):
     clocks = sampler.stop() if rank == 0 else None
     launches, evals, real_moves = eng.launches() - l0, eng.evals() - ev0, eng.moves - mv0
     note(f"timed region: {K} steps in {dev_ms:.1f} ms device / {wall * 1e3:.1f} ms wall, {evals} evaluations")
+    if args.dump_outputs:
+        # the root tables MctsBatch.results() hands a caller after the last timed wave, games in batch order
+        res = [sp.mcts.results() for sp in eng.sp]
+        out = {k: np.concatenate([r[k] for r in res]) for k in ("visits", "root_value", "best_q", "best_action", "total_visits")}
+        out["root_priors"] = np.concatenate([sp.mcts.root_priors() for sp in eng.sp])
+        dump_outputs(args.dump_outputs, out, rank, world)
+        note(f"outputs of the last timed step written to {args.dump_outputs}")
 
     # ---- e2e: the same waves through the host-buffer tensor boundary (float32 "s"), wall clock --------
     Ke = min(K, args.e2e_steps)
@@ -1186,7 +1227,7 @@ def main():
     os.dup2(2, 1)  # fd 1 -> stderr for native libraries and stray prints
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 20 for selfplay, 30 for playout)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="selfplay", choices=["selfplay", "playout"])
@@ -1208,12 +1249,19 @@ def main():
     ap.add_argument("--dim", type=int, default=256)
     ap.add_argument("--nn-batch", type=int, default=NN_BATCH)
     ap.add_argument("--fake-net", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32/float64, "
+                         "at most 64 MB; same arguments, same inputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the outputs of --impl ours")
+    if args.steps is None:
+        args.steps = 30 if args.workload == "playout" else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     BOARD = args.board
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.workload == "playout":
-        if args.steps == 20:
-            args.steps = 30
         return run_reference_playout(args) if args.impl == "reference" else run_playout(args)
     global ROLLOUTS
     if BOARD == 9:  # BASELINE configs[4]: 9x9, 16384 concurrent games, 400 rollouts per move

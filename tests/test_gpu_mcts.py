@@ -1,6 +1,6 @@
 """GPU parity of the batched tree search (CUDA, through the C ABI) against the oracle: the C
-restatement (oracle/mcts_oracle.c, itself pinned exactly to the compiled reference search) and,
-when oracle/_ref is present, the UNMODIFIED reference search itself.  One search thread, fixed
+restatement (oracle/mcts_oracle.c, itself pinned exactly to the compiled reference search) and the
+UNMODIFIED reference search itself (oracle/_ref when built, else its root tables stored in tests/golden).  One search thread, fixed
 rollouts per batch, rotation_flip off, deterministic fake net (oracle/fakenet.h).
 Bar (BASELINE.json north_star): root visit counts within +-1 per edge."""
 import json
@@ -27,7 +27,27 @@ def fake_actor(mcts, n):
     return actor
 
 
-def run_gpu_vs_cpu(sc, use_ref, tol=1):
+class GoldenMcts:
+    """the compiled reference search's root tables of one game, replayed from tests/golden/mcts_<name>.json
+    (scripts/gen_golden.py: steps in [move][game] order, games played on the reference's own choice)"""
+
+    def __init__(self, steps, g, G, n, evals):
+        self.steps, self.P1, self.evals = steps[g::G], n * n + 1, evals
+        self.k = 0
+
+    def act(self, state):
+        st = self.steps[self.k]
+        self.k += 1
+        v = np.full(self.P1, -1, np.int64)
+        for a, c in st["visits"].items():
+            v[int(a)] = c
+        return {"visits": v, "total_visits": st["total_visits"], "best_action": st["best_action"]}
+
+    def num_evals(self):
+        return self.evals
+
+
+def run_gpu_vs_cpu(sc, use_ref, tol=1, golden=None):
     import elf_b200
 
     n, G = sc["n"], sc["G"]
@@ -44,7 +64,10 @@ def run_gpu_vs_cpu(sc, use_ref, tol=1):
             assert s.forward(acts[g])
         assert gb.forward(acts).all()
     mc = elf_b200.MctsBatch(gb, rotation_flip=0, **sc["opts"])
-    cpu = [(oracles.RefMcts if use_ref else oracles.OracleMcts)(n, **sc["opts"]) for _ in range(G)]
+    if golden is not None:
+        cpu = [GoldenMcts(golden["steps"], g, G, n, golden["num_evals"] if g == 0 else 0) for g in range(G)]
+    else:
+        cpu = [(oracles.RefMcts if use_ref else oracles.OracleMcts)(n, **sc["opts"]) for _ in range(G)]
     actor = fake_actor(mc, n)
     worst, exact = 0, 0
     for mv in range(sc["moves"]):
@@ -59,11 +82,13 @@ def run_gpu_vs_cpu(sc, use_ref, tol=1):
             exact += d == 0
             assert d <= tol, f"visits differ by {d} at move {mv} game {g}"
             assert res["total_visits"][g] == rr["total_visits"]
-            assert res["root_value"][g] == np.float32(rr["root_value"])
+            if golden is None:  # the stored tables hold visits, totals and the chosen move only
+                assert res["root_value"][g] == np.float32(rr["root_value"])
             if d == 0:
                 # an exact most-visited tie resolves in the reference's container order, on the device too
                 assert res["best_action"][g] == rr["best_action"], f"move {mv} game {g}"
-                assert abs(res["best_q"][g] - rr["best_q"]) < 1e-5
+                if golden is None:
+                    assert abs(res["best_q"][g] - rr["best_q"]) < 1e-5
             acts[g] = rr["best_action"]
             assert states[g].forward(acts[g])
         assert gb.forward(acts).all()
@@ -83,9 +108,12 @@ def test_gpu_search_vs_restatement(name):
 
 @pytest.mark.parametrize("name", sorted(SCENARIOS))
 def test_gpu_search_vs_reference(name):
-    if not oracles.have_ref(SCENARIOS[name]["n"]):
-        pytest.skip("oracle/_ref not built")
-    run_gpu_vs_cpu(SCENARIOS[name], use_ref=True)
+    """against the compiled reference search when oracle/_ref is built, else against its stored root tables"""
+    if oracles.have_ref(SCENARIOS[name]["n"]):
+        run_gpu_vs_cpu(SCENARIOS[name], use_ref=True)
+    else:
+        golden = json.load(open(os.path.join(GOLD, f"mcts_{name}.json")))
+        run_gpu_vs_cpu(SCENARIOS[name], use_ref=False, golden=golden)
 
 
 def test_gpu_search_many_games_batched():

@@ -1,12 +1,12 @@
 """SGF reader (elf_b200/sgf.py) against the reference's reader and its own gtests.
 
-* known answers of /root/reference/src_cpp/elfgames/go/sgf/sgf_test.cc (9x9, MiniGo-derived game
+* known answers of ELF's src_cpp/elfgames/go/sgf/sgf_test.cc (9x9, MiniGo-derived game
   records): coordinates, header fields, every move replayable, the "miracle final board";
 * field-by-field parity with the compiled reference Sgf class (oracle/_ref, ref_sgf_parse) on those
   records, on synthetic records made from oracle playouts (with blanks, comments, escapes, passes,
-  off-board letters) and, when the reference tree is present, on its 19x19 ladder_suite records.
+  off-board letters) and, from stored results (tests/golden), on a sample of its 19x19 ladder_suite records.
 """
-import glob
+import json
 import os
 import random
 
@@ -113,8 +113,13 @@ def test_main_line_of_a_tree():
 
 
 # ---- parity with the compiled reference reader ------------------------------------------------
-def same_as_reference(text, n):
-    want = oracles.ref_sgf_parse(text, n)
+REF_PARSE = object()
+
+
+def same_as_reference(text, n, want=REF_PARSE):
+    """``want``: what the reference's reader returned for ``text`` (default: ask the compiled reference)"""
+    if want is REF_PARSE:
+        want = oracles.ref_sgf_parse(text, n)
     try:
         got = sgf.Sgf.loads(text, n)
     except ValueError:
@@ -184,17 +189,19 @@ def test_reader_matches_reference_on_synthetic_records(oracle_lib):
     assert total > 5000
 
 
-LADDER = "/root/reference/ladder_suite/ladder"
+LADDER = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sgf_ladder_suite.json")
 
 
-@needs_ref19
-@pytest.mark.skipif(not os.path.isdir(LADDER), reason="reference tree not present (GPU box)")
 def test_reader_matches_reference_on_ladder_suite(oracle_lib):
-    files = sorted(glob.glob(LADDER + "/*.sgf"))
-    assert len(files) > 100
-    for f in files:
-        text = open(f, errors="replace").read()
-        k = same_as_reference(text, 19)
+    """a sample of ELF's ladder_suite records (tests/golden) with the reference reader's results stored beside
+    them; when the compiled reference is present it is asked again and must still agree with the stored data"""
+    records = json.load(open(LADDER))["records"]
+    assert len(records) > 25
+    for r in records:
+        text, f = r["text"], r["name"]
+        if oracles.have_ref(19):
+            assert oracles.ref_sgf_parse(text, 19) == r["reference"], f
+        k = same_as_reference(text, 19, r["reference"])
         assert k > 20, f
         # every record is a legal 19x19 game for the board restatement as well
         rec = sgf.Sgf.loads(text)
