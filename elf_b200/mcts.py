@@ -129,12 +129,15 @@ class MctsBatch(RefStreamSearch):
                                                                  self.cpad if cpad is None else cpad))
 
     def leaf_count(self):
+        """the number of leaves of the last wave (waits for the context stream); after
+        ``select(wait=False)`` it also becomes the row count ``leaf_info`` / ``expand_backup`` use"""
         n = ctypes.c_int32()
         _l.check(self._lib, self._lib.elfb200_mcts_leaf_count(self._m, ctypes.byref(n)))
+        self._n = n.value
         return n.value
 
     def leaf_info(self):
-        n = self._n
+        n = self._n if self._n >= 0 else self.leaf_count()
         h = np.empty(n, np.uint64)
         g = np.empty(n, np.int32)
         p = np.empty(n, np.int32)

@@ -75,11 +75,11 @@ if __name__ == "__main__":
 
 def gen_mcts():
     """tests/golden/mcts_<scenario>.json: root visit counts of the compiled reference search."""
-    from tests.test_mcts_oracle_vs_ref import SCENARIOS, run_search
+    from tests.test_mcts_oracle_vs_ref import SCENARIOS, ref_mcts, run_search
 
     for name, sc in sorted(SCENARIOS.items()):
         n = sc["n"]
-        res, evals = run_search(sc, lambda: oracles.Ref(n), lambda: oracles.RefMcts(n, **sc["opts"]))
+        res, evals = run_search(sc, lambda: oracles.Ref(n), lambda: ref_mcts(sc))
         steps = []
         for r in res:
             v = r["visits"]
@@ -90,5 +90,21 @@ def gen_mcts():
         print("golden mcts fixture", name)
 
 
+def gen_scale_sample():
+    """tests/golden/mcts_19_scale_sample.json: the compiled reference search's root-table records (move,
+    total visits, root value, digest of visits and priors) of the 64 sampled games of
+    tests/test_gpu_search_at_scale.py.  Each game's opening comes from a generator of its own, so only the
+    sampled games are searched."""
+    from tests import test_gpu_search_at_scale as S
+
+    games = S.sample_games(4096)
+    d = {"seed": S.SEED, "opts": S.OPTS, "games": games.tolist(), "tables": S.reference_records(games)}
+    with open(S.GOLD, "w") as f:
+        json.dump(d, f)
+    print("golden mcts fixture 19_scale_sample")
+
+
 if __name__ == "__main__" and (len(sys.argv) == 1 or "mcts" in sys.argv):
     gen_mcts()
+if __name__ == "__main__" and (len(sys.argv) == 1 or "scale" in sys.argv):
+    gen_scale_sample()

@@ -101,10 +101,11 @@ class EmuSearch(RefStreamSearch):
     def leaf_count(self):
         k = ctypes.c_int32()
         _l.check(self._lib, self._lib.elfb200_mcts_leaf_count(self._m, ctypes.byref(k)))
+        self._n = k.value
         return k.value
 
     def leaf_info(self):
-        n = self._n
+        n = self._n if self._n >= 0 else self.leaf_count()
         h, g, p = np.empty(n, np.uint64), np.empty(n, np.int32), np.empty(n, np.int32)
         self.leaf_d4 = np.empty(n, np.int32)
         _l.check(self._lib, self._lib.elfb200_mcts_leaf_info(self._m, h.ctypes.data, g.ctypes.data, p.ctypes.data,

@@ -629,3 +629,67 @@ def feature_net(x, num_actions):
     p = np.exp(z)
     p /= p.sum(1, keepdims=True)
     return p.astype(np.float32), np.tanh(x @ w2).astype(np.float32)
+
+
+class IntNet:
+    """deterministic test net computed FROM THE PLANES whose answer is the same bits on the device
+    (torch, any batch shape, any GEMM summation order, TF32 or not) and on the host (numpy).
+
+    logits = planes (0/1) . W with W integer in [-7, 7]: every partial sum is an integer of magnitude
+    below 18*361*7 < 2^24, exact in float32 in any order.  pi = TABLE[bucket(logit)] with TABLE[k] =
+    2^((k - levels + 1) / 4), left unnormalised like ``fakenet`` (pi2response renormalises over the
+    legal moves); few buckets -> bit-equal probabilities among the legal moves of almost every reply, as a
+    half-precision network produces them.  v = clamp(planes . w_v, -1023, 1023) / 1024, exact."""
+
+    def __init__(self, n, levels=24, seed=0):
+        rng = np.random.default_rng([n, levels, seed])
+        K, A = 18 * n * n, n * n + 1
+        self.n, self.levels = n, int(levels)
+        self.W = rng.integers(-7, 8, size=(K, A)).astype(np.int64)
+        self.w_v = rng.integers(-7, 8, size=K).astype(np.int64)
+        self.table = np.exp2((np.arange(levels) - (levels - 1)) / 4.0).astype(np.float32)
+        # a reply's logits spread with the standard deviation of a sum of ~n*n uniform terms (4.3 n):
+        # the middle bucket sits at 0 and `levels` buckets cover about +-2 of those deviations
+        self.den = int(np.ceil(4 * 4.3 * n))
+        self._dev = {}
+
+    def _bucket(self, logit, floordiv, clip):
+        return clip(floordiv(logit * self.levels, self.den) + self.levels // 2, 0, self.levels - 1)
+
+    def numpy(self, x):
+        """x: planes [m, 18, n, n] (any dtype holding 0/1) -> (pi float32 [m, A], v float32 [m])"""
+        x = np.asarray(x).reshape(len(x), -1)
+        assert ((x == 0) | (x == 1)).all()
+        if not hasattr(self, "_W64"):  # integer sums far below 2^53: float64 products are exact
+            self._W64 = np.concatenate([self.W, self.w_v[:, None]], 1).astype(np.float64)
+        z = np.rint(x.astype(np.float64) @ self._W64).astype(np.int64)
+        logit, lv = z[:, :-1], z[:, -1]
+        pi =self.table[self._bucket(logit, np.floor_divide, np.clip)]
+        v = (np.clip(lv, -1023, 1023).astype(np.float32) / np.float32(1024)).astype(np.float32)
+        return pi.astype(np.float32), v
+
+    def __call__(self, feats, hashes=None):
+        """the RefMcts / OracleMcts callback signature"""
+        return self.numpy(feats)
+
+    def torch(self, s):
+        """s: CUDA planes, float32 NCHW [m, 18, n, n] or 16-bit NHWC [m, n, n, cpad] (planes in
+        channels 0..17) -> (pi float32 [m, A], v float32 [m]) on s's device"""
+        import torch
+
+        dev = s.device
+        if dev not in self._dev:
+            W = torch.from_numpy(np.concatenate([self.W, self.w_v[:, None]], 1).astype(np.float32)).to(dev)
+            self._dev[dev] = (W, torch.from_numpy(self.table).to(dev))
+        W, table = self._dev[dev]
+        x = s.float() if s.dim() == 4 and s.shape[1] == 18 and s.shape[-1] == self.n else s[..., :18].float().permute(0, 3, 1, 2)
+        z = torch.round(x.reshape(x.shape[0], -1) @ W).to(torch.int64)
+        logit, lv = z[:, :-1], z[:, -1]
+        pi = table[self._bucket(logit, lambda a, b: torch.div(a, b, rounding_mode="floor"), torch.clamp)]
+        v =torch.clamp(lv, -1023, 1023).to(torch.float32) / 1024
+        return pi.contiguous(), v.contiguous()
+
+
+def int_net(n, levels=24, seed=0):
+    """see IntNet"""
+    return IntNet(n, levels, seed)

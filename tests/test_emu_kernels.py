@@ -781,7 +781,8 @@ def test_expand_half_size_sort_network_on_late_positions(emu, oracle_lib):
     assert (mc.errors() == 0).all()
 
 
-@pytest.mark.parametrize("name", ["9_noprior_ties", "9_rounding_ties", "9_superko_in_tree"])
+@pytest.mark.parametrize("name", ["9_noprior_ties", "9_rounding_ties", "9_superko_in_tree", "9_equal_priors",
+                                  "19_equal_priors"])
 def test_puct_ties_resolve_in_the_reference_container_order(emu, name, lane_order):
     """k_select's uct_tie_break: exactly equal PUCT scores (no prior term; priors lost in the rounding of
     q) go to the first tied edge in the order of the reference's unordered_map, also when that edge lies
@@ -789,8 +790,10 @@ def test_puct_ties_resolve_in_the_reference_container_order(emu, name, lane_orde
     COMPILED reference search's, move after move (twin of test_gpu_mcts.py::test_gpu_search_vs_reference).
     9_superko_in_tree: a recapture two plies below the root repeats a position of the game -- a terminal
     node inside the tree; the 9x9 search used to miss such a repetition when the move captured and the
-    matching record was scanned by a lane beyond the board's rows (found by scripts/emu_fuzz_streams.py)"""
-    from tests.test_mcts_oracle_vs_ref import SCENARIOS, scenario_openings
+    matching record was scanned by a lane beyond the board's rows (found by scripts/emu_fuzz_streams.py).
+    *_equal_priors: a net with bit-equal probabilities among the legal moves (std_sort_ties, k_expand<N, true>);
+    priors bit-identical too"""
+    from tests.test_mcts_oracle_vs_ref import SCENARIOS, ref_mcts, scenario_net, scenario_openings, search_options
 
     sc = SCENARIOS[name]
     n, G = sc["n"], sc["G"]
@@ -807,15 +810,24 @@ def test_puct_ties_resolve_in_the_reference_container_order(emu, name, lane_orde
             acts[g] = int(fixed[g][t]) if fixed is not None else int(rng.choice(idx))
             assert s.forward(acts[g])
         assert gb.forward(acts).all()
-    mc = emu.EmuSearch(gb, rotation_flip=0, **sc["opts"])
-    refs = [oracles.RefMcts(n, **sc["opts"]) for _ in range(G)]
-    actor = fake_actor(mc, n)
+    mc = emu.EmuSearch(gb, rotation_flip=0, **search_options(sc), **sc["opts"])
+    refs = [ref_mcts(sc) for _ in range(G)]
+    net = scenario_net(sc)
+    if net is None:
+        actor = fake_actor(mc, n)
+    else:
+        def actor(batch):
+            pi, v = net(None, mc.leaf_info()[0])
+            return {"pi": torch.from_numpy(pi), "V": torch.from_numpy(v)}
     for mv in range(sc["moves"]):
         res = mc.act(actor)
+        pri = mc.root_priors()
         acts = np.empty(G, np.int32)
         for g in range(G):
             rr = refs[g].act(states[g])
             np.testing.assert_array_equal(res["visits"][g], rr["visits"], err_msg=f"move {mv} game {g}")
+            has = rr["visits"] >= 0
+            np.testing.assert_array_equal(pri[g][has], rr["prior"][has], err_msg=f"priors, move {mv} game {g}")
             assert res["total_visits"][g] == rr["total_visits"] and res["best_action"][g] == rr["best_action"]
             assert res["root_value"][g] == np.float32(rr["root_value"]) and abs(res["best_q"][g] - rr["best_q"]) < 1e-5
             acts[g] = rr["best_action"]
@@ -870,3 +882,76 @@ def test_equal_priors_follow_std_sort(emu, n, quant, lane_order):
             assert gb.forward(acts).all()
             mc.advance(acts)
         assert (mc.errors() == 0).all(), mc.errors()
+
+
+def test_async_leaf_count_then_leaf_info(emu):
+    """the asynchronous wave from Python: select(wait=False) -> leaf_count() -> leaf_info() (the hashes of
+    exactly the counted leaves) -> fake net -> expand_backup checked against the known count; root tables
+    equal the synchronous search's"""
+    n, G = 9, 4
+    opts = dict(num_rollouts=40, num_rollouts_per_batch=5, virtual_loss=1, persistent_tree=1, c_puct=1.5)
+
+    def make():
+        gb = emu.emu_batch(G, n)
+        rng = np.random.default_rng(4)
+        for _ in range(12):
+            lm = gb.legal_mask()[:, :-1]
+            assert gb.forward(np.array([int(rng.choice(np.flatnonzero(r))) for r in lm], np.int32)).all()
+        return gb, emu.EmuSearch(gb, rotation_flip=0, **opts)
+
+    (gb0, m0), (gb1, m1) = make(), make()
+    for _ in range(3):
+        r0 = m0.act(fake_actor(m0, n))
+        m1.begin_move()
+        for _ in range(m1.waves_per_move):
+            assert m1.select(wait=False).shape[0] == m1.max_leaves
+            k = m1.leaf_count()
+            h = m1.leaf_info()[0]
+            assert len(h) == k
+            if k == 0:
+                m1.expand_backup(None, None)
+                continue
+            pi, v = oracles.fakenet(h, n * n + 1)
+            with pytest.raises(AssertionError):  # fewer rows than the known count
+                m1.expand_backup(torch.from_numpy(pi[: k - 1]), torch.from_numpy(v[: k - 1]))
+            m1.expand_backup(torch.from_numpy(pi), torch.from_numpy(v))
+        r1 = m1.results()
+        for key in ("visits", "best_action", "total_visits", "root_value", "best_q"):
+            np.testing.assert_array_equal(r0[key], r1[key])
+        np.testing.assert_array_equal(m0.root_priors(), m1.root_priors())
+        a = r0["best_action"]
+        for gb, m in ((gb0, m0), (gb1, m1)):
+            assert gb.forward(a).all()
+            m.advance(a)
+    assert m1.eval_count() == m0.eval_count() and (m1.errors() == 0).all()
+
+
+def test_bench_search_twin_on_the_kernels(emu):
+    """small-G twin of tests/test_gpu_search_at_scale.py on the emulated kernels: 19x19 games with the seeded
+    openings of 0..150 plies, binary16 NHWC leaf batches, the asynchronous leaf count, batches padded with NaN
+    replies, the plane-reading IntNet (equal probabilities everywhere, std_sort_ties=1), a fresh root and a
+    move on the kept tree -- root tables equal the COMPILED reference's, priors bit for bit"""
+    from tests import test_gpu_search_at_scale as S
+
+    if not oracles.have_ref(S.N):
+        pytest.skip("compiled reference (oracle/_ref) not available")
+    G = 4
+    opts = dict(S.OPTS, num_rollouts=48)
+    games = np.arange(G)
+    gb = emu.emu_batch(G, S.N)
+    S.play_openings(gb, 0)
+    legal = gb.legal_mask()[:, :-1].sum(1)
+    assert legal.min() < 256 < legal.max(), legal  # both sort networks of k_expand
+    net = S.net()
+    want = S.reference_records(games, net, opts)
+    mc = emu.EmuSearch(gb, rotation_flip=0, feature_format="f16", cpad=24, std_sort_ties=1, **opts)
+    actor = S.PaddedActor(net, [mc], batchsize=12)
+    dup = 0
+    for move in range(S.MOVES):
+        S.async_wave_search(mc, actor)
+        res = mc.results()
+        dup += S.compare_sample(res, mc.root_priors(), games, want, move)
+        assert gb.forward(res["best_action"]).all()
+        mc.advance(res["best_action"])
+    assert (mc.errors() == 0).all(), mc.errors()
+    assert actor.padded > 0 and dup >= G

@@ -43,7 +43,56 @@ SCENARIOS = {
     "9_superko_in_tree": dict(n=9, G=1, moves=3, open_plies=64, openings="mcts_superko_opening_9.json",
                               opts=dict(num_rollouts=96, num_rollouts_per_batch=8, virtual_loss=1, persistent_tree=1, c_puct=5.0,
                                         komi=5.5, ply_pass_enabled=30)),
+    # a net whose probabilities sit on a grid of 1/quant (bit-equal values among the legal moves of almost
+    # every reply, as a half-precision network answers): the reference's pi2response leaves equal values in
+    # the order of libstdc++'s std::sort, which the searches reproduce with std_sort_ties (the compiled
+    # reference always sorts that way and takes no such option)
+    "9_equal_priors": dict(n=9, G=3, moves=5, open_plies=20, quant=64, std_sort_ties=1,
+                           opts=dict(num_rollouts=96, num_rollouts_per_batch=6, virtual_loss=1, persistent_tree=1, c_puct=1.5,
+                                     ply_pass_enabled=40)),
+    "19_equal_priors": dict(n=19, G=1, moves=3, open_plies=40, quant=256, std_sort_ties=1,
+                            opts=dict(num_rollouts=128, num_rollouts_per_batch=8, virtual_loss=1, persistent_tree=1, c_puct=1.5)),
 }
+
+
+def quantised_fakenet(n, quant):
+    """the fake net with its probabilities on a grid of 1/quant: bit-equal values everywhere, as a
+    half-precision network produces them"""
+    def net(feats, hashes):
+        pi, v = oracles.fakenet(hashes, n * n + 1)
+        return (np.floor(pi * np.float32(quant)) / np.float32(quant)).astype(np.float32), v
+
+    return net
+
+
+def scenario_net(sc):
+    """the scenario's network as a (feats, hashes) -> (pi, v) callback; None = the built-in fake net"""
+    return quantised_fakenet(sc["n"], sc["quant"]) if "quant" in sc else None
+
+
+def search_options(sc):
+    """keyword arguments beyond sc["opts"] of the restatement, emulated and device searches of a scenario
+    (the compiled reference always sorts like std::sort and takes no std_sort_ties)"""
+    return {"std_sort_ties": sc["std_sort_ties"]} if "std_sort_ties" in sc else {}
+
+
+def ref_mcts(sc):
+    """the compiled reference search of a scenario"""
+    return oracles.RefMcts(sc["n"], callback=scenario_net(sc), **sc["opts"])
+
+
+def oracle_mcts(sc, lib=None):
+    """the C restatement of the search for a scenario"""
+    return oracles.OracleMcts(sc["n"], lib=lib, callback=scenario_net(sc), **search_options(sc), **sc["opts"])
+
+
+def duplicate_prior_share(results):
+    """share of root tables (run_search results) in which two root edges have bit-equal priors"""
+    dup = 0
+    for r in results:
+        p = r["prior"][r["visits"] >= 0]
+        dup += len(np.unique(p)) < len(p)
+    return dup / len(results)
 
 
 def scenario_openings(sc):
@@ -92,10 +141,12 @@ def test_restatement_equals_reference(name, oracle_lib):
     if not oracles.have_ref(n):
         pytest.skip("oracle/_ref not built (needs /root/reference)")
     oa, ob = [], []
-    a, ea = run_search(sc, lambda: oracles.Ref(n), lambda: oracles.RefMcts(n, **sc["opts"]), orders=oa)
-    b, eb = run_search(sc, lambda: oracles.Oracle(n, oracle_lib), lambda: oracles.OracleMcts(n, lib=oracle_lib, **sc["opts"]),
+    a, ea = run_search(sc, lambda: oracles.Ref(n), lambda: ref_mcts(sc), orders=oa)
+    b, eb = run_search(sc, lambda: oracles.Oracle(n, oracle_lib), lambda: oracle_mcts(sc, oracle_lib),
                        forced=[r["best_action"] for r in a], orders=ob)
     assert ea == eb
+    if "quant" in sc:  # the scenario reaches the equal-prior tie-breaks at the root
+        assert duplicate_prior_share(a) >= 0.9, duplicate_prior_share(a)
     for i, (ra, rb) in enumerate(zip(a, b)):
         # the most-visited move is the first maximum in the reference's container order: same move, ties included
         assert ra["best_action"] == rb["best_action"], i
@@ -113,7 +164,7 @@ def test_restatement_equals_golden(name, oracle_lib):
     gold = json.load(open(path))
     sc = SCENARIOS[name]
     n = sc["n"]
-    b, eb = run_search(sc, lambda: oracles.Oracle(n, oracle_lib), lambda: oracles.OracleMcts(n, lib=oracle_lib, **sc["opts"]),
+    b, eb = run_search(sc, lambda: oracles.Oracle(n, oracle_lib), lambda: oracle_mcts(sc, oracle_lib),
                        forced=[st["best_action"] for st in gold["steps"]])
     assert eb == gold["num_evals"]
     assert len(b) == len(gold["steps"])
@@ -158,7 +209,7 @@ def test_selected_prefix_property(name, oracle_lib):
     sc = SCENARIOS[name]
     n = sc["n"]
     states = opening(n, sc["G"], sc["open_plies"], lambda: oracles.Oracle(n, oracle_lib), scenario_openings(sc))
-    ms = [oracles.OracleMcts(n, lib=oracle_lib, **sc["opts"]) for _ in range(sc["G"])]
+    ms = [oracle_mcts(sc, oracle_lib) for _ in range(sc["G"])]
     for _ in range(sc["moves"]):
         for s, m in zip(states, ms):
             s.forward(m.act(s)["best_action"])
@@ -168,16 +219,6 @@ def test_selected_prefix_property(name, oracle_lib):
     if name.endswith("_ties"):  # these scenarios are there for the container-order tie-break
         ties, beyond = sum(m.tie_stats()[0] for m in ms), sum(m.tie_stats()[1] for m in ms)
         assert ties > 0 and (beyond > 0 or name == "9_rounding_ties"), (ties, beyond)
-
-
-def quantised_fakenet(n, quant):
-    """the fake net with its probabilities on a grid of 1/quant: bit-equal values everywhere, as a
-    half-precision network produces them"""
-    def net(feats, hashes):
-        pi, v = oracles.fakenet(hashes, n * n + 1)
-        return (np.floor(pi * np.float32(quant)) / np.float32(quant)).astype(np.float32), v
-
-    return net
 
 
 @pytest.mark.parametrize("quant", [16, 256, 4096])
